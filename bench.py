@@ -189,6 +189,40 @@ def run_reference(args):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
+DUMP_PARAM_SAMPLE = 1 << 22  # parameters --dump-outputs writes: a fixed, seeded sample (16 MB as float32) of the 223 M
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, spec, store):
+    """--dump-outputs: what a caller of the timed step receives from its last run, as DIR/<name>.npy in float32/float64 --
+    the three losses, every logged metric, the joint encoder's hidden states, and the updated parameters sampled at fixed
+    seeded positions of their reference-named, name-sorted concatenation -- so that two builds run with the same arguments
+    (hence the same inputs) can be compared output for output.  Reads buffers the next step overwrites: call it first."""
+    import re
+    import numpy as np
+    arrays = {"loss_parts": np.array([float(x) for x in spec.loss_parts], dtype=np.float64)}
+    for k, v in spec.metrics.items():
+        arrays["metric_" + re.sub(r"[^0-9A-Za-z]+", "_", k).strip("_")] = torch.as_tensor(v).detach().double().cpu().numpy()
+    for k, v in spec.model.encoder_hidden_states.items():
+        arrays[f"hidden_{k}"] = v.detach().float().cpu().numpy()
+    params = store.to_tf_dict("p")
+    names = sorted(params)
+    offs = np.cumsum([0] + [params[n].numel() for n in names])
+    idx = np.unique(np.random.default_rng(0).integers(0, offs[-1], DUMP_PARAM_SAMPLE))
+    owner = np.searchsorted(offs, idx, side="right") - 1
+    sample = np.empty(idx.size, dtype=np.float32)
+    for i in np.unique(owner):
+        sel = owner == i
+        sample[sel] = params[names[i]].reshape(-1).numpy()[idx[sel] - offs[i]]
+    arrays["params_sample"] = sample
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
 def run_ours(args):
     from merlot_b200 import _lib as L
     from merlot_b200.train import DataParallel, model_fn_builder, synthetic_batch
@@ -236,6 +270,9 @@ def run_ours(args):
     sync_all()
     launches = int(lib.merlot_launch_count())
     log("timed region done")
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, spec, store)
+        log(f"outputs of the last timed step written to {args.dump_outputs}")
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if dist is not None:
         dist.dist.all_reduce(ms, op=dist.dist.ReduceOp.MAX)
@@ -578,7 +615,13 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch override for --config 1/4/5")
     ap.add_argument("--stem", default="patch", choices=["patch", "hybrid"],
                     help="hybrid: merlot.yaml as shipped (ResNet-lite stem before the ViT); default = the north star's patch embedding")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (headline workload only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != 2):
+        ap.error("--dump-outputs applies to the headline workload (--impl ours, --config 2)")
     global STEM
     STEM = args.stem
     if args.impl == "reference":

@@ -65,6 +65,37 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert "workload" in d["config"]
 
 
+def test_bench_dump_outputs_are_float_seeded_and_bounded(tmp_path, tiny_cfg):
+    """`bench.py --dump-outputs DIR`: float32/float64 .npy files within 64 MB, identical for identical state, and the parameter
+    sample reads the reference-named, name-sorted concatenation at the positions the fixed seed draws."""
+    import sys
+    from types import SimpleNamespace
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    st = ParamStore(tiny_cfg, device="cpu")
+    st.init_reference(seed=0)
+    spec = SimpleNamespace(loss_parts=(torch.tensor(2.5), torch.tensor(0.75), torch.tensor(1.25)),
+                           metrics={"lang/loss": torch.tensor(2.5), "contr/lang_to_viz": torch.tensor(0.5), "learning_rate": 3e-7},
+                           model=SimpleNamespace(encoder_hidden_states={"viz": torch.randn(2, 14, 128), "lang": torch.randn(2, 32, 128)}))
+    for d in ("a", "b"):
+        bench.write_outputs(str(tmp_path / d), spec, st)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) and "params_sample.npy" in names and "loss_parts.npy" in names
+    assert "metric_contr_lang_to_viz.npy" in names and "hidden_viz.npy" in names
+    total = 0
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), n
+        total += a.nbytes
+    assert total <= 64 << 20
+    assert np.load(tmp_path / "a" / "loss_parts.npy").tolist() == [2.5, 0.75, 1.25]
+    params = st.to_tf_dict("p")
+    flat = np.concatenate([params[k].reshape(-1).numpy() for k in sorted(params)])
+    idx = np.unique(np.random.default_rng(0).integers(0, flat.size, bench.DUMP_PARAM_SAMPLE))
+    assert np.array_equal(np.load(tmp_path / "a" / "params_sample.npy"), flat[idx])
+
+
 def test_pairwise_partner_words_equal_the_reference_mask():
     """disable_pairwise_lang_attn (model/modeling.py:160-168): the attention kernels never see an [S, S] mask -- every row
     derives its partners as two bit ranges per 32-position word (csrc/attention_tcgen05.cu: span_word / pair_lo_of / pair_word).
